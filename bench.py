@@ -42,6 +42,8 @@ ALG_BYTES = {"glcm": 5 + 8 * 24, "glrlm": 5 + 8 * 16, "glszm": 5 + 8 * 16, "gldm
 CLASSES = ("glcm", "glrlm", "glszm", "gldm", "ngtdm")
 METRIC = "voxels/s full-texture voxel-based"
 RTOL, ATOL = 1e-5, 1e-9
+# --dump-outputs: 75 float64 maps at 100 000 sampled voxels = 60 MB, within the 64 MB a dump may take
+DUMP_VOXELS, DUMP_SEED = 100_000, 7
 
 
 def synth_volume(n, kind):
@@ -282,7 +284,27 @@ def parity_of(outs, z0, vox, feats):
             "oracle": "oracle/_ref compiled reference _cmatrices + oracle/features_np.py"}
 
 
-def measure_suite(ctx, vol, steps, warmup, classes=CLASSES, oracle=None, check_determinism=True, sample_clocks=False):
+def dump_outputs(ctx, outs, z0, n, out_dir):
+    """--dump-outputs: the maps {class: [F, nz, Y, X]} of the last timed step at a fixed, seeded sample of voxels of the n^3
+    volume (the same sample for every run with the same --size) -> out_dir/<class>.npy, float64 [F, voxels]; every rank
+    contributes the voxels of its slab, rank 0 writes"""
+    import torch
+    vox = torch.from_numpy(sample_voxels(n, min(DUMP_VOXELS, n ** 3), DUMP_SEED).astype(np.int64)).to(ctx.dev)
+    nz = next(iter(outs.values())).shape[1]
+    mine = (vox[0] >= z0) & (vox[0] < z0 + nz)
+    zl = (vox[0] - z0).clamp(0, nz - 1)
+    if ctx.rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+    for c, t in outs.items():
+        s = torch.where(mine, t[:, zl, vox[1], vox[2]], 0.0)
+        if ctx.world > 1:
+            ctx.dist.all_reduce(s)
+        if ctx.rank == 0:
+            np.save(os.path.join(out_dir, f"{c}.npy"), s.cpu().numpy())
+
+
+def measure_suite(ctx, vol, steps, warmup, classes=CLASSES, oracle=None, check_determinism=True, sample_clocks=False,
+                  dump_dir=None):
     """device-resident timing of the fused kernels over `vol` (levels), z-slabs over the ranks"""
     import torch
     from pyradiomics_b200 import _lib, distributed as D, voxel
@@ -341,7 +363,9 @@ def measure_suite(ctx, vol, steps, warmup, classes=CLASSES, oracle=None, check_d
     per_class_ms = {c: float(np.mean([a.elapsed_time(b) for a, b in ev[c]])) for c in classes}
     res = {"value": float(np.prod(vol.shape)) * steps / (ms * 1e-3), "ms_per_step": ms / steps, "per_class_ms": per_class_ms,
            "launches": launches[0], "clocks": clocks, "nz": nz}
-    # ---- outside the timed region: bit-reproducibility and the sampled oracle comparison
+    # ---- outside the timed region: the dumped outputs, bit-reproducibility and the sampled oracle comparison
+    if dump_dir is not None:
+        dump_outputs(ctx, outs, z0, vol.shape[0], dump_dir)
     if check_determinism:
         same = True
         for c in classes:
@@ -541,7 +565,7 @@ def run_b200(args):
             oracle_s = (vox_s, feats_s)
 
     ctx = Ctx(args)
-    main = measure_suite(ctx, vol, args.steps, args.warmup, oracle=oracle, sample_clocks=True)
+    main = measure_suite(ctx, vol, args.steps, args.warmup, oracle=oracle, sample_clocks=True, dump_dir=args.dump_outputs)
     value, per_class_ms, nz = main["value"], main["per_class_ms"], main["nz"]
     Z = args.size
 
@@ -618,7 +642,13 @@ def main():
     ap.add_argument("--cpu-workers", type=int, default=64)
     ap.add_argument("--cpu-voxels-per-worker", type=int, default=96)
     ap.add_argument("--parity-voxels", type=int, default=20480)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the feature maps of the last timed step, at a fixed sample of voxels, as DIR/<class>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

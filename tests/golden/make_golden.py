@@ -456,7 +456,58 @@ def resample_goldens():
     np.savez_compressed(os.path.join(HERE, "resample_cases.npz"), **out)
 
 
+def reference_runs():
+    """what the tests compare with the compiled reference extensions and classes, so that they need neither ->
+    reference_runs.json:
+    (a) port_trials: sha256 digests (helpers.digest) of every matrix the reference _cmatrices returns on the seeded
+        trials of helpers.port_trials (null where the reference refuses the trial's angles);
+    (b) argument_errors: the exception type the reference _cmatrices raises for each malformed call of
+        test_plugin_host_logic_cpu.BAD_CALLS;
+    (c) large_roi_shape: the reference _cshape's (surface area, volume, diameters) of test_shape_gpu's 96^3 ellipsoid;
+    (d) feature_names: getFeatureNames() of the reference's feature classes."""
+    import importlib
+
+    import build_ref
+    sys.path[:0] = [os.path.join(HERE, ".."), os.path.join(HERE, "..", "..")]
+    import helpers
+    from test_plugin_host_logic_cpu import BAD_CALLS
+    from test_shape_gpu import large_roi_case
+
+    cm = build_ref.load()
+    trials = []
+    for trial, *args in helpers.port_trials():
+        if args[1].sum() == 0:
+            trials.append(None)
+            continue
+        try:
+            trials.append([helpers.digest(a) for a in helpers.port_trial_outputs(cm, *args)])
+        except RuntimeError:
+            trials.append(None)
+    errors = {}
+    img, msk = np.ones((4, 5, 6), np.int32), np.ones((4, 5, 6), bool)
+    for what, call in BAD_CALLS.items():
+        try:
+            call(cm, img, msk)
+        except Exception as e:
+            errors[what] = type(e).__name__
+    m, sp = large_roi_case()
+    sa, vol, dia = build_ref.load("_cshape").calculate_coefficients(m, sp)
+    names = {}
+    for mod, cls in (("glcm", "RadiomicsGLCM"), ("glrlm", "RadiomicsGLRLM"), ("glszm", "RadiomicsGLSZM"), ("gldm", "RadiomicsGLDM"),
+                     ("ngtdm", "RadiomicsNGTDM"), ("firstorder", "RadiomicsFirstOrder"), ("shape", "RadiomicsShape"),
+                     ("shape2D", "RadiomicsShape2D")):
+        names[mod] = getattr(importlib.import_module(f"radiomics.{mod}"), cls).getFeatureNames()
+    out = {"port_trials": trials, "argument_errors": errors,
+           "large_roi_shape": {"surface_area": float(sa), "volume": float(vol), "diameters": [float(v) for v in dia]},
+           "feature_names": names}
+    json.dump(out, open(os.path.join(HERE, "reference_runs.json"), "w"), indent=0, sort_keys=True)
+    print("reference runs:", sum(t is not None for t in trials), "port trials,", len(errors), "argument errors")
+
+
 if __name__ == "__main__":
+    if "--reference-runs-only" in sys.argv:
+        reference_runs()
+        sys.exit(0)
     if "--segment-variants-only" in sys.argv:
         segment_goldens_variants()
         sys.exit(0)

@@ -36,3 +36,31 @@ def test_bench_line_contract(path):
 
 def test_at_least_one_line_is_committed():
     assert LINES
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_from_run_to_run(tmp_path):
+    """--dump-outputs writes one float64 [features, voxels] array per class, 64 MB at most, and two runs with the same
+    arguments write the same values; --steps is the number of timed steps the line reports"""
+    import subprocess
+    import sys
+
+    import numpy as np
+    n_features = {"glcm": 24, "glrlm": 16, "glszm": 16, "gldm": 14, "ngtdm": 5}
+    dumps = []
+    for run, steps in enumerate((1, 2)):
+        out = tmp_path / f"run{run}"
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", str(steps), "--warmup", "1",
+                            "--size", "40", "--no-e2e", "--no-secondary", "--no-cpu-baseline", "--no-numa-bind",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert p.returncode == 0, p.stderr[-2000:]
+        assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == steps
+        files = sorted(os.listdir(out))
+        assert files == sorted(f"{c}.npy" for c in n_features)
+        assert sum(os.path.getsize(out / f) for f in files) <= 64 << 20
+        d = {f[:-4]: np.load(out / f) for f in files}
+        for c, a in d.items():
+            assert a.dtype == np.float64 and a.shape == (n_features[c], 40 ** 3)
+        dumps.append(d)
+    for c in n_features:
+        assert np.array_equal(dumps[0][c], dumps[1][c], equal_nan=True), c

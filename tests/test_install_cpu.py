@@ -1,29 +1,64 @@
-"""CPU test of the drop-in boundary: `pyradiomics_b200.install()` against the REFERENCE's own registry (imported where
-it lies, with stand-ins for SimpleITK / pywt / pykwalify: oracle/ref_harness.py) -- the feature-class dictionary, the
-per-module `cMatrices` rebinding (SURVEY.md 8b) and `cShape` keeping `calculate_coefficients2D` reachable for
-radiomics.shape2D (reference radiomics/shape2D.py:99).  No CUDA call is made."""
+"""CPU test of the drop-in boundary: `pyradiomics_b200.install()` against a package registry built like the reference's --
+the feature-class dictionary, the per-module `cMatrices` rebinding (SURVEY.md 8b) and `cShape` keeping
+`calculate_coefficients2D` reachable for radiomics.shape2D (reference radiomics/shape2D.py:99) -- and the feature names
+against the reference classes' (tests/golden/reference_runs.json).  No CUDA call is made."""
 import importlib
+import json
 import os
 import sys
 
 import pytest
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "radiomics")), reason="the reference tree is not on this box")
+from helpers import GOLDEN
+
+# A package laid out like the reference's radiomics: getFeatureClasses() imports the class modules once and caches the
+# dictionary it returns (radiomics/__init__.py:104-117); the extensions are package attributes that every class module
+# binds by name at import time (`from radiomics import base, cMatrices` in glcm.py, `... cShape` in shape.py / shape2D.py).
+STANDIN = {
+    "__init__.py": '''
+import importlib
+import inspect
+import types
+
+cMatrices = types.ModuleType("_cmatrices")
+cShape = types.ModuleType("_cshape")
+cShape.calculate_coefficients = lambda *a: None
+cShape.calculate_coefficients2D = lambda *a: None
+_featureClasses = None
+
+
+def getFeatureClasses():
+    global _featureClasses
+    if _featureClasses is None:
+        _featureClasses = {}
+        for mod in ("firstorder", "glcm", "gldm", "glrlm", "glszm", "ngtdm", "shape", "shape2D"):
+            for _, cls in inspect.getmembers(importlib.import_module(__name__ + "." + mod), inspect.isclass):
+                if "RadiomicsFeaturesBase" in [b.__name__ for b in cls.__mro__[1:]]:
+                    _featureClasses[mod] = cls
+    return _featureClasses
+''',
+    "base.py": "class RadiomicsFeaturesBase:\n    pass\n",
+}
+for _mod, _ext in (("firstorder", "cMatrices"), ("glcm", "cMatrices"), ("gldm", "cMatrices"), ("glrlm", "cMatrices"),
+                   ("glszm", "cMatrices"), ("ngtdm", "cMatrices"), ("shape", "cShape"), ("shape2D", "cShape")):
+    STANDIN[f"{_mod}.py"] = (f"from radiomics_standin import base, {_ext}\n\n\n"
+                             f"class Radiomics{_mod}(base.RadiomicsFeaturesBase):\n    pass\n")
 
 
 @pytest.fixture(scope="module")
-def rad():
-    import types
-    import ref_harness
-    # radiomics.getFeatureClasses() imports EVERY module of the package, radiomics.scripts (the CLI) among them: stand-ins
-    # for what the CLI imports and this image lacks
-    if "ruamel" not in sys.modules:
-        ru, ry = types.ModuleType("ruamel"), types.ModuleType("ruamel.yaml")
-        ry.YAML = type("YAML", (), {"__init__": lambda self, *a, **k: None})
-        ru.yaml = ry
-        sys.modules["ruamel"], sys.modules["ruamel.yaml"] = ru, ry
-    return ref_harness.load_reference()
+def rad(tmp_path_factory):
+    root = tmp_path_factory.mktemp("standin")
+    pkg = root / "radiomics_standin"
+    pkg.mkdir()
+    for name, src in STANDIN.items():
+        (pkg / name).write_text(src)
+    sys.path.insert(0, str(root))
+    try:
+        yield importlib.import_module("radiomics_standin")
+    finally:
+        sys.path.remove(str(root))
+        for m in [m for m in sys.modules if m == "radiomics_standin" or m.startswith("radiomics_standin.")]:
+            del sys.modules[m]
 
 
 def test_install_registers_classes_and_rebinds_cmatrices(rad):
@@ -52,15 +87,14 @@ def test_install_registers_classes_and_rebinds_cmatrices(rad):
         cshape.no_such_function
 
 
-def test_feature_names_and_docstrings_match_the_reference_classes(rad):
-    """reference tests/test_docstrings.py: every get<Name>FeatureValue has a docstring; names equal the reference's"""
+def test_feature_names_and_docstrings_match_the_reference_classes():
+    """reference tests/test_docstrings.py: every get<Name>FeatureValue has a docstring; names (and their deprecation flags)
+    equal the reference classes' getFeatureNames()"""
     from pyradiomics_b200 import featureclasses as FC
+    ref = json.load(open(os.path.join(GOLDEN, "reference_runs.json")))["feature_names"]
     for name in ("glcm", "glrlm", "glszm", "gldm", "ngtdm", "firstorder", "shape", "shape2D"):
-        ref_cls = getattr(importlib.import_module(f"{rad.__name__}.{name}"), {"glcm": "RadiomicsGLCM", "glrlm": "RadiomicsGLRLM",
-                          "glszm": "RadiomicsGLSZM", "gldm": "RadiomicsGLDM", "ngtdm": "RadiomicsNGTDM",
-                          "firstorder": "RadiomicsFirstOrder", "shape": "RadiomicsShape", "shape2D": "RadiomicsShape2D"}[name])
         ours = {**FC.FEATURE_CLASSES, **FC.NEXT_CLASSES}[name]
-        assert ours.getFeatureNames() == ref_cls.getFeatureNames()
+        assert ours.getFeatureNames() == ref[name]
         for f in ours.getFeatureNames():
             assert getattr(ours, f"get{f}FeatureValue").__doc__
 

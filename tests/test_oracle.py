@@ -8,7 +8,7 @@ import pytest
 
 import cmatrices_oracle as O
 import pipeline as PL
-from helpers import GOLDEN, assert_maps_close, ref_map, voxel_goldens
+from helpers import GOLDEN, assert_maps_close, digest, port_trial_outputs, port_trials, ref_map, voxel_goldens
 
 CASES = ["brain1", "brain2", "breast1", "lung1", "lung2"]
 
@@ -18,56 +18,20 @@ def seg():
     return np.load(os.path.join(GOLDEN, "segment_cases.npz")), json.load(open(os.path.join(GOLDEN, "segment_expect.json")))
 
 
-def _ref_module():
-    import build_ref
-    try:
-        return build_ref.load()
-    except ImportError:
-        return None
-
-
 def test_port_equals_compiled_reference():
     """bit-exact agreement of oracle/cmatrices_port.c with the gcc-built reference _cmatrices on
-    random 2-D/3-D inputs, segment and voxel mode, several distances / force2D."""
-    R = _ref_module()
-    if R is None:
-        pytest.skip("oracle/_ref not built and /root/reference absent")
-    rng = np.random.default_rng(3)
+    random 2-D/3-D inputs, segment and voxel mode, several distances / force2D: every matrix and angle table
+    against the digest of the reference's (tests/golden/reference_runs.json)."""
+    ref = json.load(open(os.path.join(GOLDEN, "reference_runs.json")))["port_trials"]
     n = 0
-    for trial in range(40):
-        nd = int(rng.choice([2, 3]))
-        shp = tuple(int(s) for s in (rng.integers(1, 9, nd) if trial % 3 else rng.integers(3, 8, nd)))
-        Ng = int(rng.integers(1, 9))
-        img = rng.integers(1, Ng + 1, shp).astype(np.int32)
-        msk = rng.random(shp) > float(rng.choice([0, 0.2, 0.6]))
-        if msk.sum() == 0:
+    for trial, *args in port_trials():
+        if ref[trial] is None:                       # empty ROI, or angles the reference refuses
             continue
-        dist = np.array([[1], [1, 2], [2], [1, 3]][trial % 4])
-        f2 = int(trial % 5 == 0 and nd == 3)
-        f2d = int(rng.integers(0, nd))
-        try:
-            ra = R.calculate_glcm(img, msk, dist, Ng, f2, f2d)
-            rr = R.calculate_glrlm(img, msk, Ng, max(shp), f2, f2d)
-        except RuntimeError:
-            continue
-        pa = O.calculate_glcm(img, msk, dist, Ng, f2, f2d)
-        assert np.array_equal(ra[0], pa[0]) and np.array_equal(ra[1], pa[1])
-        pr = O.calculate_glrlm(img, msk, Ng, max(shp), f2, f2d)
-        assert np.array_equal(rr[0], pr[0]) and np.array_equal(rr[1], pr[1])
-        Ns = int(msk.sum())
-        assert np.array_equal(R.calculate_glszm(img, msk, Ng, Ns, f2, f2d), O.calculate_glszm(img, msk, Ng, Ns, f2, f2d))
-        assert np.array_equal(R.calculate_ngtdm(img, msk, dist, Ng, f2, f2d), O.calculate_ngtdm(img, msk, dist, Ng, f2, f2d))
-        assert np.array_equal(R.calculate_gldm(img, msk, dist, Ng, 1, f2, f2d), O.calculate_gldm(img, msk, dist, Ng, 1, f2, f2d))
-        vox = np.array(np.where(msk)).astype(np.int32)
-        if vox.shape[1] < 2:
-            continue
-        r = int(rng.integers(1, 3))
-        assert np.array_equal(R.calculate_glcm(img, msk, dist, Ng, f2, f2d, r, vox)[0], O.calculate_glcm(img, msk, dist, Ng, f2, f2d, r, vox)[0])
-        assert np.array_equal(R.calculate_glrlm(img, msk, Ng, max(shp), f2, f2d, r, vox)[0], O.calculate_glrlm(img, msk, Ng, max(shp), f2, f2d, r, vox)[0])
-        assert np.array_equal(R.calculate_glszm(img, msk, Ng, Ns, f2, f2d, r, vox), O.calculate_glszm(img, msk, Ng, Ns, f2, f2d, r, vox))
-        assert np.array_equal(R.calculate_ngtdm(img, msk, dist, Ng, f2, f2d, r, vox), O.calculate_ngtdm(img, msk, dist, Ng, f2, f2d, r, vox))
-        assert np.array_equal(R.calculate_gldm(img, msk, dist, Ng, 0, f2, f2d, r, vox), O.calculate_gldm(img, msk, dist, Ng, 0, f2, f2d, r, vox))
-        n += 1
+        got = [digest(a) for a in port_trial_outputs(O, *args)]
+        assert len(got) == len(ref[trial])
+        for k, (g, r) in enumerate(zip(got, ref[trial])):
+            assert g == r, (trial, k)
+        n += len(got) == 12
     assert n > 20
 
 

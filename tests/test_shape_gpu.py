@@ -1,5 +1,5 @@
 """Shape path on the GPU through the C ABI: CUDA marching cubes / all-pairs diameters / voxel moments
-against the reference's outputs (committed goldens) and, where it travelled, the compiled reference."""
+against the reference's outputs (committed goldens)."""
 import json
 import os
 import sys
@@ -68,25 +68,23 @@ def test_deprecated_features_on_request_and_voxel_mode_refused():
         featureclasses.RadiomicsShape(img, msk, voxelBased=True).execute()
 
 
-def test_large_roi_against_compiled_reference():
-    """96^3 ellipsoid with holes (~5e4 mesh vertices, 1e9 vertex pairs) against oracle/_ref/_cshape when it
-    travelled with the snapshot; otherwise against the NumPy brute force on a vertex subsample-free small case."""
-    sys.path.insert(0, os.path.join(HERE, "..", "oracle"))
-    import build_ref
-    try:
-        cs = build_ref.load("_cshape")
-    except ImportError:
-        pytest.skip("compiled reference _cshape not available")
-    from pyradiomics_b200 import cshape
+def large_roi_case():
+    """96^3 ellipsoid with holes (~5e4 mesh vertices, 1e9 vertex pairs) and its spacing"""
     rng = np.random.default_rng(5)
     z, y, x = np.meshgrid(np.arange(96), np.arange(96), np.arange(96), indexing="ij")
     m = (((z - 47.3) / 40) ** 2 + ((y - 48.2) / 33) ** 2 + ((x - 46.1) / 44) ** 2 < 1.0) & (rng.random(z.shape) > 0.02)
-    sp = np.array((1.7, 0.9, 1.2))
-    ref = cs.calculate_coefficients(m, sp)
+    return m, np.array((1.7, 0.9, 1.2))
+
+
+def test_large_roi_against_compiled_reference():
+    """large_roi_case() against the compiled reference _cshape's outputs (tests/golden/reference_runs.json)"""
+    from pyradiomics_b200 import cshape
+    ref = json.load(open(os.path.join(G, "reference_runs.json")))["large_roi_shape"]
+    m, sp = large_roi_case()
     sa, vol, dia = cshape.calculate_coefficients(m, sp)
-    assert sa == pytest.approx(ref[0], rel=1e-11)
-    assert vol == pytest.approx(ref[1], rel=1e-11)
-    assert tuple(dia) == tuple(ref[2])
+    assert sa == pytest.approx(ref["surface_area"], rel=1e-11)
+    assert vol == pytest.approx(ref["volume"], rel=1e-11)
+    assert tuple(dia) == tuple(ref["diameters"])
 
 
 SHAPE2D = ["disc", "noise", "sparse", "touching_border", "single", "checker", "ring"]
