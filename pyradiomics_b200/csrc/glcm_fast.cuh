@@ -556,6 +556,7 @@ RB_HD uint32_t glcm_fast_voxel_phaseA(const uint8_t* w, int ws, uint32_t* eq, in
   for (int k = 0; k < GLCM_NF; k++) out[k] = acc.n_ok ? acc.sum[k] * inv : NAN;
   out[G_Imc2] = acc.n_imc2 ? acc.sum[G_Imc2] / acc.n_imc2 : NAN;
   if (acc.ja_nan) out[G_JointAverage] = NAN;
+  if (P.n_roi_levels < 2) out[G_MCC] = 1.0;      // flat ROI: 1 for every centre, with or without pairs (glcm.py:702)
   return acc.tasks;
 }
 

@@ -464,6 +464,7 @@ RB_HD void glcm_voxel(const uint16_t* w, const VoxParams& P, double* out, int* s
     bool ok = glcm_angle_features<ECAP, WCAP, NJCAP, double>(E, n, val, P, f, status);
     if (E.overflow) { ok = false; if (status) *status |= 2; }
     for (int k = 0; k < GLCM_NF; k++) out[k] = ok ? f[k] : NAN;
+    if (P.n_roi_levels < 2) out[G_MCC] = 1.0;    // flat ROI: 1 for every centre, with or without pairs (glcm.py:702)
     return;
   }
   double sum[GLCM_NF]; int cnt[GLCM_NF];
@@ -486,6 +487,7 @@ RB_HD void glcm_voxel(const uint16_t* w, const VoxParams& P, double* out, int* s
   for (int k = 0; k < GLCM_NF; k++) out[k] = cnt[k] ? sum[k] / cnt[k] : NAN;
   // JointAverage is a plain mean over the kept angles (glcm.py:292): NaN propagates
   if (ja_nan) out[G_JointAverage] = NAN;
+  if (P.n_roi_levels < 2) out[G_MCC] = 1.0;
 }
 
 // --------------------------------------------------------------------------------------------
@@ -680,6 +682,16 @@ RB_HD void gldm_voxel(const uint16_t* w, const VoxParams& P, double* out) {
 }
 
 // --------------------------------------------------------------------------------------------
+// A product rounded on its own, never contracted into a following subtraction: where numpy's i*p_i - j*p_j is exactly 0
+// (equal products) a fused multiply-add leaves the rounding error of one product, and a zero denominator becomes ~1e-17.
+RB_HD double mul_rn(double a, double b) {
+#ifdef __CUDA_ARCH__
+  return __dmul_rn(a, b);
+#else
+  return a * b;
+#endif
+}
+
 template <int WCAP>
 RB_HD void ngtdm_voxel(const uint16_t* w, const VoxParams& P, double* out) {
   const WinGeom G(P);
@@ -711,7 +723,7 @@ RB_HD void ngtdm_voxel(const uint16_t* w, const VoxParams& P, double* out) {
     for (int b = 0; b < n; b++) {
       double pb = cnt[b] / Nvp, ib = val[b], d = ia - ib;
       con += pa * pb * d * d;
-      busy_den += fabs(ia * pa - ib * pb);
+      busy_den += fabs(mul_rn(ia, pa) - mul_rn(ib, pb));
       cpx += fabs(d) * (pa * s[a] + pb * s[b]) / (pa + pb);
       str += (pa + pb) * d * d;
     }

@@ -11,7 +11,8 @@ import pytest
 
 import cmatrices_oracle as O
 import pipeline as PL
-from helpers import assert_maps_close, binned, ref_map, voxel_goldens
+from helpers import (adversarial_windows, assert_maps_close, binned, mcc_angle_numpy, random_window, ref_map, slot_angles,
+                     voxel_goldens)
 from pyradiomics_b200 import _lib
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -151,104 +152,6 @@ def test_glcm_fast_math_equals_generic_math_on_host(emul, kind):
         assert np.allclose(fast[k], gen[k], rtol=1e-7, atol=atol, equal_nan=True), f
 
 
-def _slot_angles():
-    """the fast path's processing order of the 13 distance-1 angles: reference order (cmatrices.c:843-860), stably
-    regrouped by the number of moving dimensions (glcm_fast_build_tables)"""
-    ang = [(z, y, x) for z in (1, 0, -1) for y in (1, 0, -1) for x in (1, 0, -1)][:13]
-    return [a for want in (1, 2, 3) for a in ang if sum(v != 0 for v in a) == want]
-
-
-def _mcc_angle_numpy(w27, a):
-    """second largest |eigenvalue| of P / sqrt(px py) for one angle of a 3x3x3 window (LAPACK), and the node count"""
-    W = w27.reshape(3, 3, 3)
-    P = np.zeros((256, 256))
-    for i in range(3):
-        for j in range(3):
-            for k in range(3):
-                ii, jj, kk = i + a[0], j + a[1], k + a[2]
-                if 0 <= ii < 3 and 0 <= jj < 3 and 0 <= kk < 3 and W[i, j, k] and W[ii, jj, kk]:
-                    P[W[i, j, k], W[ii, jj, kk]] += 1
-                    P[W[ii, jj, kk], W[i, j, k]] += 1
-    nz = P.sum(1) > 0
-    n = int(nz.sum())
-    if n < 2:
-        return None, n
-    Pn = P[nz][:, nz]
-    px = Pn.sum(1)
-    # connected graphs only (the solver is never asked otherwise)
-    reach = np.zeros(n, bool); reach[0] = True
-    for _ in range(n):
-        reach |= (Pn[reach].sum(0) > 0)
-    if not reach.all():
-        return None, n
-    ev = np.sort(np.abs(np.linalg.eigvalsh(Pn / np.sqrt(np.outer(px, px)))))[::-1]
-    return float(ev[1]), n
-
-
-def _windows(rng, it):
-    K = int(rng.integers(2, 33))
-    mode = it % 5
-    if mode == 0:
-        w = rng.integers(1, K + 1, 27)
-    elif mode == 1:
-        g = np.cumsum(rng.integers(-1, 2, 27)) + rng.integers(0, 2, 27)
-        w = g - g.min() + 1
-    elif mode == 2:
-        zz, yy, xx = np.meshgrid(range(3), range(3), range(3), indexing="ij")
-        c = rng.normal(size=3) * K / 4
-        w = np.round(c[0] * zz + c[1] * yy + c[2] * xx + rng.normal(size=(3, 3, 3)) * 0.7).reshape(27)
-        w = w - w.min() + 1
-    elif mode == 3:
-        w = rng.integers(1, K + 1, 27)
-        w[rng.random(27) < 0.2] = 0
-    else:
-        w = rng.integers(1, 33, 27)              # i.i.d. uniform on 32 levels: the 13..18-level graphs of the headline volume
-    return np.ascontiguousarray(np.clip(w, 0, 32), dtype=np.uint8)
-
-
-def _adversarial_windows():
-    """symmetric / near-bipartite / repeated-eigenvalue level graphs (what a fixed Lanczos start vector could miss)"""
-    out = []
-    W = np.zeros((3, 3, 3), int)
-    # mirror-symmetric windows along every axis (repeated eigenvalues by symmetry)
-    base = np.arange(1, 10).reshape(3, 3)
-    for ax in range(3):
-        for shift in (0, 9):
-            w = np.stack([base + shift, base + 9 - shift // 9, base + shift], axis=ax)
-            out.append(w.reshape(27))
-    # long even / odd cycles and paths through the 27 positions (snake order): bipartite or one odd cycle
-    snake = []
-    for z in range(3):
-        ys = range(3) if z % 2 == 0 else range(2, -1, -1)
-        for y in ys:
-            xs = range(3) if (y + z) % 2 == 0 else range(2, -1, -1)
-            for x in xs:
-                snake.append((z, y, x))
-    for period in (2, 3, 4, 5, 7, 9, 13, 17, 18):
-        w = np.zeros((3, 3, 3), int)
-        for k, (z, y, x) in enumerate(snake):
-            w[z, y, x] = 1 + k % period
-        out.append(w.reshape(27))
-        out.append(w.transpose(2, 1, 0).reshape(27))
-        out.append(w.transpose(1, 0, 2).reshape(27))
-    # checkerboards with one defect (bipartite plus a single self-pair / odd cycle)
-    zz, yy, xx = np.meshgrid(range(3), range(3), range(3), indexing="ij")
-    cb = 1 + (zz + yy + xx) % 2
-    for k in range(27):
-        w = cb.reshape(27).copy()
-        w[k] = 3 + k % 3
-        out.append(w)
-    # star graphs: one hub level everywhere, distinct leaves
-    for hub_every in (2, 3):
-        w = np.arange(1, 28)
-        w[::hub_every] = 31
-        out.append(w)
-    # two dense clusters joined by one pair (near-degenerate second eigenvalue close to 1)
-    w = np.where(np.arange(27) < 13, 1 + np.arange(27) % 3, 10 + np.arange(27) % 3)
-    out.append(w)
-    return [np.ascontiguousarray(np.clip(w, 0, 32), dtype=np.uint8) for w in out]
-
-
 @pytest.fixture(scope="module")
 def emul_dyn():
     """the same device math with the task-sized eigenvalue search (LZ_EIG_EXACT_STATIC=0)"""
@@ -266,15 +169,15 @@ def test_eigen_task_solvers_against_lapack(emul, emul_dyn):
     on random / structured / holed / adversarial windows, against numpy's eigvalsh -- both in fp64 throughout: 1e-9"""
     emul.emul_glcm_solve_window_cls.restype = C.c_double
     emul.emul_glcm_lanczos_axis.restype = C.c_double
-    slots = _slot_angles()
+    slots = slot_angles()
     rng = np.random.default_rng(11)
     worst = {"dense": 0.0, "lanczos": 0.0, "lanczos_small": 0.0}
     count = {"dense": 0, "lanczos": 0, "lanczos_small": 0}
-    wins = [_windows(rng, it) for it in range(1500)] + _adversarial_windows()
+    wins = [random_window(rng, it) for it in range(1500)] + adversarial_windows()
     for w in wins:
         p = w.ctypes.data_as(C.c_void_p)
         for s, a in enumerate(slots):
-            ref, n = _mcc_angle_numpy(w, a)
+            ref, n = mcc_angle_numpy(w, a)
             if ref is None:
                 continue
             d = emul.emul_glcm_solve_window_cls(p, s, 32, -1)
@@ -312,11 +215,11 @@ def test_eigen_task_solvers_against_lapack(emul, emul_dyn):
 def test_phaseA_graph_scan_against_bruteforce(emul):
     """glcm_graph_scan (one breadth-first sweep over class masks: connected? bipartite?) on the level graphs of random /
     structured / holed windows, all 13 angles"""
-    slots = _slot_angles()
+    slots = slot_angles()
     rng = np.random.default_rng(5)
     seen = {(c, b): 0 for c in (0, 1) for b in (0, 1)}
     for it in range(8000):
-        w = _windows(rng, it)
+        w = random_window(rng, it)
         a = slots[it % 13]
         prs = [(i * 9 + j * 3 + k, (i + a[0]) * 9 + (j + a[1]) * 3 + k + a[2]) for i in range(3) for j in range(3) for k in range(3)
                if 0 <= i + a[0] < 3 and 0 <= j + a[1] < 3 and 0 <= k + a[2] < 3]

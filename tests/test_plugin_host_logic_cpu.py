@@ -12,7 +12,7 @@ import pytest
 
 import cmatrices_oracle as O
 import pipeline as PL
-from helpers import GOLDEN
+from helpers import GOLDEN, check_segment_baseline_columns, check_segment_variant_runs
 from pyradiomics_b200 import cmatrices, featureclasses as FC, image as I
 
 CLASSES = ("glcm", "glrlm", "glszm", "gldm", "ngtdm")
@@ -60,38 +60,13 @@ def _columns():
 
 @pytest.mark.parametrize("cname", CLASSES)
 def test_plugin_classes_over_oracle_matrices_match_every_baseline_column(oracle_device, cname):
-    cases, base, extra, masks = _columns()
-    cols = dict(base[cname])
-    cols.update(extra[cname])
-    assert len(cols) == (35 if cname in ("glcm", "glrlm") else 30)      # (the *_combined columns exist for GLCM / GLRLM only)
-    for test, e in cols.items():
-        c = e["case"]
-        img = cases[c + "_image"]
-        m = masks[test + "_mask"] if test + "_mask" in masks.files else cases[c + "_mask"]
-        if "normalize" in e:
-            n = e["normalize"]
-            img = (img.astype(np.float64) - n["mean"]) / n["std"] * n["scale"]
-        obj = FC.FEATURE_CLASSES[cname](I.ArrayImage(img, cases[c + "_spacing"]), I.ArrayImage(m.astype(np.uint8), cases[c + "_spacing"]),
-                                        **e["settings"])
-        got = obj.execute()
-        assert set(got) == set(e["features"]), (test, set(got) ^ set(e["features"]))
-        for f, v in e["features"].items():
-            assert abs(float(got[f]) - v) <= 1e-9 * max(abs(v), 1e-12), (cname, test, f, float(got[f]), v)
+    check_segment_baseline_columns(cname)
 
 
 @pytest.mark.parametrize("cname", CLASSES)
 def test_plugin_classes_over_oracle_matrices_match_reference_runs_of_other_settings(oracle_device, cname):
     """weighting norms (featureclasses._weights), several distances, asymmetric GLCM, force2D, binCount, gldm_a"""
-    cases = np.load(os.path.join(GOLDEN, "segment_cases.npz"))
-    expect = json.load(open(os.path.join(GOLDEN, "segment_expect_variants.json")))[cname]
-    for test, e in expect.items():
-        c = e["case"]
-        sp = cases[c + "_spacing"]
-        got = FC.FEATURE_CLASSES[cname](I.ArrayImage(cases[c + "_image"], sp), I.ArrayImage(cases[c + "_mask"].astype(np.uint8), sp),
-                                        **e["settings"]).execute()
-        assert set(got) == set(e["features"]), (test, set(got) ^ set(e["features"]))
-        for f, v in e["features"].items():
-            assert np.isclose(float(got[f]), v, rtol=1e-9, atol=1e-12, equal_nan=True), (cname, test, e["settings"], f, float(got[f]), v)
+    check_segment_variant_runs(cname)
 
 
 @pytest.mark.parametrize("case", ["brain1", "brain2", "breast1", "lung1", "lung2"])

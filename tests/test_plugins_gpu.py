@@ -10,7 +10,8 @@ import torch
 
 import filters_np as FN
 import pipeline as PL
-from helpers import GOLDEN, assert_maps_close, ref_map, voxel_goldens
+from helpers import (GOLDEN, assert_maps_close, check_segment_baseline_columns, check_segment_variant_runs, ref_map,
+                     voxel_goldens)
 from pyradiomics_b200 import featureclasses as FC, image as I, imageoperations as IO
 
 pytestmark = pytest.mark.gpu
@@ -74,7 +75,20 @@ def test_processed_matrices_match_reference_golden(seg, case):
         assert np.abs(P - cases[f"{case}_{cname}_P"]).max() < 1e-3
 
 
-@pytest.mark.parametrize("name,z,kw", voxel_goldens(), ids=[g[0] for g in voxel_goldens()])
+@pytest.mark.parametrize("cname", list(FC.FEATURE_CLASSES))
+def test_segment_features_match_every_baseline_column(cname):
+    """the 160 baseline columns without resampling (resegmented masks, normalisation included) over the CUDA matrices, at
+    1e-9: the host logic is pinned on the oracle's matrices (test_plugin_host_logic_cpu.py), so a failure here is the kernels'"""
+    check_segment_baseline_columns(cname)
+
+
+@pytest.mark.parametrize("cname", list(FC.FEATURE_CLASSES))
+def test_segment_features_match_reference_runs_of_other_settings(cname):
+    """weighting norms, several distances, asymmetric GLCM, force2D, binCount, gldm_a over the CUDA matrices, at 1e-9"""
+    check_segment_variant_runs(cname)
+
+
+@pytest.mark.parametrize("name,z,kw", voxel_goldens(extra=True), ids=[g[0] for g in voxel_goldens(extra=True)])
 def test_voxel_based_plugin_maps_match_reference(name, z, kw):
     sp = z["spacing"]
     img = I.ArrayImage(z["image"], sp)

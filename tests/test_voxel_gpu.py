@@ -25,15 +25,36 @@ def _maps_host(cname, lev, Ng, nlev, spacing=(1, 1, 1), **kw):
     return dict(zip(_lib.feature_names(cname), out))
 
 
-@pytest.mark.parametrize("name,z,kw", voxel_goldens(), ids=[g[0] for g in voxel_goldens()])
+# voxelx_image2d is left to test_plugins_gpu.py: how a 2-D image maps onto one plane (spacing, force2D axis) is decided in
+# featureclasses, not in the kernels' C ABI
+GOLDENS = [g for g in voxel_goldens(extra=True) if g[0] != "image2d"]
+
+
+@pytest.mark.parametrize("name,z,kw", GOLDENS, ids=[g[0] for g in GOLDENS])
 def test_golden_maps_from_the_reference(name, z, kw):
-    lev, levels, Ng = binned(z, kw)
-    lev = np.where(z["mask"], lev, 0)
-    kw2 = {k: v for k, v in kw.items() if k not in ("binWidth", "binCount")}
+    kw2 = {k: v for k, v in kw.items() if k not in ("binWidth", "binCount", "maskedKernel")}
+    sp = z["spacing"][::-1]
+    if kw.get("maskedKernel", True):
+        lev, levels, Ng = binned(z, kw)
+        lev = np.where(z["mask"], lev, 0)
+        for cname in _lib.CLASSES:
+            got = _maps_host(cname, lev, Ng, len(levels), spacing=sp, **kw2)
+            for f, arr in got.items():
+                assert_maps_close(arr, ref_map(z, cname, f), f"{name}/{cname}/{f}")
+        return
+    # unmasked kernel (maskedKernel=False): the whole image is binned and seen by the windows, the ROI only selects the
+    # centre voxels -- the device API's `centers`
+    lev, _, levels, Ng = PL.bin_image(z["image"], np.ones(z["mask"].shape, bool), kw.get("binWidth", 25), kw.get("binCount"))
+    img = torch.as_tensor(np.ascontiguousarray(lev, dtype=np.int32)).cuda()
+    packed, _ = voxel.pack_levels(img, torch.ones_like(img), Ng)
+    centers = torch.as_tensor(np.ascontiguousarray(z["mask"], dtype=np.uint8)).cuda()
+    s = _lib.make_settings(Ng, len(levels), spacing_zyx=sp, **kw2)
+    m = z["mask"].astype(bool)
     for cname in _lib.CLASSES:
-        got = _maps_host(cname, lev, Ng, len(levels), spacing=z["spacing"][::-1], **kw2)
-        for f, arr in got.items():
-            assert_maps_close(arr, ref_map(z, cname, f), f"{name}/{cname}/{f}")
+        out = voxel.voxel_features(cname, packed, s, centers=centers).cpu().numpy()
+        for k, f in enumerate(_lib.feature_names(cname)):
+            assert (out[k][~m] == 0).all(), f"{name}/{cname}/{f}: initValue outside the ROI"
+            assert_maps_close(out[k][m], ref_map(z, cname, f).reshape(m.shape)[m], f"{name}/{cname}/{f}")
 
 
 def _random_volume(kind, shape, seed):
@@ -83,8 +104,9 @@ def test_slab_and_reflection_properties_at_scale(cname):
     flipped = voxel.voxel_features(cname, lev.flip(2).contiguous(), s).flip(3)
     a, b = whole.cpu().numpy(), flipped.cpu().numpy()
     assert np.isfinite(a).all()
-    # MCC eigen-tasks keep their Lanczos vectors in float32: reflection-invariant to ~1e-7 only
-    assert np.allclose(a, b, rtol=2e-6 if cname == "glcm" else 1e-9, atol=1e-12)
+    # a reflection reorders the level-graph nodes of the fp64 eigen-solves (and their floating-point sums): MCC moves in
+    # the last bits only
+    assert np.allclose(a, b, rtol=1e-9, atol=1e-11 if cname == "glcm" else 1e-12)
 
 
 def test_tensor_api_matches_host_api():
@@ -109,7 +131,9 @@ def test_glcm_fast_path_equals_generic_kernel(kind, monkeypatch):
     monkeypatch.delenv("B200_RADIOMICS_FORCE_GENERIC")
     names = _lib.feature_names("glcm")
     for k, f in enumerate(names):
-        # MCC / Imc2 of near-degenerate angles are rounding noise in every implementation
+        # the generic kernel's MCC is a bisection on the eigenvalues of M M^T followed by a square root near 0, good to
+        # ~1e-7 absolute (the fast path's MCC is held to 1e-9 against LAPACK in test_voxel_fastpath_edges_gpu.py); Imc1 / Imc2
+        # of near-independent margins are rounding noise in every implementation
         atol = 1e-6 if f in ("MCC", "Imc2", "Imc1") else 1e-9
         assert np.allclose(fast[k], gen[k], rtol=1e-7, atol=atol, equal_nan=True), f
 
